@@ -21,6 +21,8 @@ an advancing Philox state.  A "step" = one utterance per GPU (weak scaling: ever
   cpu_baseline  the oracle port (torch-CPU fp32 restatement of the reference; MLX is not installable) on the host cores, bounded sample.
 `--impl reference` times that same CPU restatement as the reference arm (rank 0 only).
 `--workload whisper|codec|qwen3` select the other BASELINE configurations (see the functions below).
+`--dump-outputs DIR` writes the waveform and durations of the last timed step as .npy files; weights, inputs and the noise state
+are seeded, so two runs with the same arguments are comparable output for output.
 """
 from __future__ import annotations
 
@@ -141,6 +143,14 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, **arrays):
+    """Write each tensor as out_dir/<name>.npy (float32 or float64), so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().cpu().numpy())
+
+
 def _union_ms(intervals):
     """Total length of the union of (start, end) intervals."""
     tot, cur_s, cur_e = 0.0, None, None
@@ -233,7 +243,7 @@ def main_kokoro(args, rank, world, local_rank):
     run_ids = model.synthesize_ids if model.use_graphs else model.forward_ids
 
     def step():
-        return run_ids(ids_d, ref_d)[0]
+        return run_ids(ids_d, ref_d)
 
     if args.ncu:
         for _ in range(2):
@@ -255,7 +265,7 @@ def main_kokoro(args, rank, world, local_rank):
         return
 
     log("model ready; capturing")
-    audio = step()
+    audio = step()[0]
     torch.cuda.synchronize(dev)
     n_samples = int(audio.shape[0])
     F = n_samples // 600
@@ -288,10 +298,13 @@ def main_kokoro(args, rank, world, local_rank):
     n0 = ops.LAUNCHES[0]
     sampler = ClockSampler(local_rank)
     sampler.start()
-    ms, audio = timed(step)
+    ms, (audio, pred_dur) = timed(step)
     clocks = sampler.stop()
     launches = ops.LAUNCHES[0] - n0
     assert audio.shape[0] == n_samples and bool(torch.isfinite(audio).all())
+    if args.dump_outputs and rank == 0:
+        # the graph path returns static buffers that the next call overwrites: copy them out before anything else runs
+        dump_outputs(args.dump_outputs, audio=audio.float(), pred_dur=pred_dur.double())
     ms_pinned, _ = timed(lambda: run_ids(ids_d, ref_d, pred_dur=dur_d, n_frames=F)[0])
     # L2 flush cost measured separately and subtracted (it is not part of the step)
     f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -469,7 +482,13 @@ def main():
                     "cudaProfilerStart/Stop (run under `ncu --profile-from-start off`); prints no bench line")
     ap.add_argument("--ncu-graph", action="store_true", help="like --ncu but the profiled step is the graph replay "
                     "(run under `ncu --profile-from-start off --graph-profiling node`)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0: audio as float32, "
+                    "pred_dur as float64) to DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "kokoro" or args.impl != "b200" or args.ncu or args.ncu_graph):
+        ap.error("--dump-outputs is available for the timed kokoro run of --impl b200 only")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

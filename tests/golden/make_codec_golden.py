@@ -15,10 +15,11 @@ import synth_params                  # noqa: E402
 
 REF = "/root/reference/mlx_audio"
 mx, nn = shim.install(precise=True)
-for name, path in (("mlx_audio", REF), ("mlx_audio.lm", f"{REF}/lm"), ("mlx_audio.lm.models", f"{REF}/lm/models"), ("mlx_audio.codec", f"{REF}/codec"),
-                   ("mlx_audio.codec.models", f"{REF}/codec/models"), ("mlx_audio.codec.models.snac", f"{REF}/codec/models/snac"),
-                   ("mlx_audio.codec.models.mimi", f"{REF}/codec/models/mimi")):
-    shim.stub_package(name, path)
+if "--replay" not in sys.argv:                                 # replaying a --live record needs no reference source
+    for name, path in (("mlx_audio", REF), ("mlx_audio.lm", f"{REF}/lm"), ("mlx_audio.lm.models", f"{REF}/lm/models"), ("mlx_audio.codec", f"{REF}/codec"),
+                       ("mlx_audio.codec.models", f"{REF}/codec/models"), ("mlx_audio.codec.models.snac", f"{REF}/codec/models/snac"),
+                       ("mlx_audio.codec.models.mimi", f"{REF}/codec/models/mimi")):
+        shim.stub_package(name, path)
 hub = types.ModuleType("huggingface_hub")
 hub.snapshot_download = hub.hf_hub_download = None
 sys.modules["huggingface_hub"] = hub
@@ -139,9 +140,12 @@ def live(n):
     import torch
     sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
     from oracle import codec as OC
-    from mlx_audio.codec.models.mimi import mimi as M
-    from mlx_audio.codec.models.mimi.modules import SeanetConfig, TransformerConfig
-    from mlx_audio.codec.models.snac import snac as S
+    from live_tape import Tape
+    tape = Tape("codec", n, sys.argv)
+    if tape.reference:
+        from mlx_audio.codec.models.mimi import mimi as M
+        from mlx_audio.codec.models.mimi.modules import SeanetConfig, TransformerConfig
+        from mlx_audio.codec.models.snac import snac as S
     worst = 0.0
     for seed in range(n):
         rng = np.random.default_rng(3000 + seed)
@@ -152,26 +156,27 @@ def live(n):
         cfg = dict(sampling_rate=24000, encoder_dim=int(rng.choice([4, 8])), encoder_rates=erates, latent_dim=None, decoder_dim=8 * 2 ** nr,
                    decoder_rates=drates, attn_window_size=None, codebook_size=int(rng.integers(16, 64)), codebook_dim=int(rng.choice([4, 8])),
                    vq_strides=vs, noise=bool(rng.integers(0, 2)), depthwise=bool(rng.integers(0, 2)))
-        model = S.SNAC(**cfg)
-        last = max(int(m.group(1)) for k, _ in shim.flat_parameters(model) if (m := re.match(r"decoder\.model\.layers\.(\d+)\.weight_g$", k)))
-        names = fill(model, rule=lambda k: "scale0.03" if k == f"decoder.model.layers.{last}.weight_g" else None)
+        if tape.reference:
+            model = S.SNAC(**cfg)
+            last = max(int(m.group(1)) for k, _ in shim.flat_parameters(model) if (m := re.match(r"decoder\.model\.layers\.(\d+)\.weight_g$", k)))
+        names = tape.value(lambda: fill(model, rule=lambda k: "scale0.03" if k == f"decoder.model.layers.{last}.weight_g" else None))
         P = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in names}
         t = int(rng.integers(1, 4)) * vs[0]
         codes = [rng.integers(0, cfg["codebook_size"], size=(2, t // st)) for st in vs]
         noises = [rng.standard_normal((2, 1, cfg["decoder_dim"] // 2 ** (i + 1))) for i in range(nr)]
-        mx.random.strict = True
-        mx.random.queue[:] = [("normal", z) for z in noises] if cfg["noise"] else []
-        audio = np.asarray(model.decode([mx.array(c) for c in codes]))
-        mx.random.queue[:] = []
-        mx.random.strict = False
+        if tape.reference:
+            mx.random.strict = True
+            mx.random.queue[:] = [("normal", z) for z in noises] if cfg["noise"] else []
+            audio = np.asarray(model.decode([mx.array(c) for c in codes]))
+            mx.random.queue[:] = []
+            mx.random.strict = False
         o = OC.snac_decode(P, [torch.as_tensor(c).long() for c in codes], cfg, [torch.as_tensor(z) for z in noises]).numpy()
-        assert audio.shape == o.shape, (audio.shape, o.shape, drates)
-        errs = [np.abs(audio - o).max()]
+        errs = [tape.err(lambda: audio, o)]
         a_in = 0.5 * rng.standard_normal((2, 1, int(rng.integers(40, 400))))
-        enc = model.encode(mx.array(a_in))
+        enc = tape.value(lambda: [np.asarray(e) for e in model.encode(mx.array(a_in))])
         oenc = OC.snac_encode(P, torch.as_tensor(a_in), cfg)
-        assert all(np.array_equal(np.asarray(e), oe.numpy()) for e, oe in zip(enc, oenc)), ("snac encode", cfg)
-        print("snac dec", drates, "enc", erates, "vq", vs, "noise", cfg["noise"], "depthwise", cfg["depthwise"], "samples", audio.shape[1], "err", float(errs[0]))
+        assert len(enc) == len(oenc) and all(np.array_equal(np.asarray(e), oe.numpy()) for e, oe in zip(enc, oenc)), ("snac encode", cfg)
+        print("snac dec", drates, "enc", erates, "vq", vs, "noise", cfg["noise"], "depthwise", cfg["depthwise"], "samples", o.shape[1], "err", float(errs[0]))
         # Mimi
         ratios = [int(v) for v in rng.choice([2, 3, 4, 5], size=int(rng.integers(2, 5)))]
         heads = int(rng.choice([1, 2, 4]))
@@ -179,26 +184,28 @@ def live(n):
              "last_ksize": int(rng.choice([3, 5])), "compress": 2, "d_model": 8 * heads, "num_heads": heads, "num_layers": int(rng.integers(1, 3)),
              "dim_feedforward": 32, "context": int(rng.integers(2, 12)), "max_period": 10000, "layer_scale": 0.01, "nq": int(rng.integers(1, 6)),
              "bins": int(rng.integers(8, 40)), "qdim": int(rng.choice([4, 8])), "upsample_stride": 2}
-        seanet = SeanetConfig(dimension=c["dimension"], channels=1, causal=True, nfilters=c["nfilters"], nresidual_layers=1, ratios=c["ratios"],
-                              ksize=c["ksize"], residual_ksize=c["residual_ksize"], last_ksize=c["last_ksize"], dilation_base=2, pad_mode="constant",
-                              true_skip=True, compress=c["compress"])
-        tr = TransformerConfig(d_model=c["d_model"], num_heads=c["num_heads"], num_layers=c["num_layers"], causal=True, norm_first=True, bias_ff=False,
-                               bias_attn=False, layer_scale=c["layer_scale"], positional_embedding="rope", use_conv_bias=True, gating=False,
-                               norm="layer_norm", context=c["context"], max_period=c["max_period"], max_seq_len=8192, kv_repeat=1,
-                               dim_feedforward=c["dim_feedforward"], conv_layout=True, use_conv_block=False, cross_attention=False, conv_kernel_size=3)
         hop = int(np.prod(ratios))
-        mm = M.Mimi(M.MimiConfig(channels=1, sample_rate=float(2 * hop * 12.5), frame_rate=12.5, renormalize=True, seanet=seanet, transformer=tr,
-                                 quantizer_nq=c["nq"], quantizer_bins=c["bins"], quantizer_dim=c["qdim"]))
-        P = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in fill(mm)}
+        if tape.reference:
+            seanet = SeanetConfig(dimension=c["dimension"], channels=1, causal=True, nfilters=c["nfilters"], nresidual_layers=1, ratios=c["ratios"],
+                                  ksize=c["ksize"], residual_ksize=c["residual_ksize"], last_ksize=c["last_ksize"], dilation_base=2, pad_mode="constant",
+                                  true_skip=True, compress=c["compress"])
+            tr = TransformerConfig(d_model=c["d_model"], num_heads=c["num_heads"], num_layers=c["num_layers"], causal=True, norm_first=True, bias_ff=False,
+                                   bias_attn=False, layer_scale=c["layer_scale"], positional_embedding="rope", use_conv_bias=True, gating=False,
+                                   norm="layer_norm", context=c["context"], max_period=c["max_period"], max_seq_len=8192, kv_repeat=1,
+                                   dim_feedforward=c["dim_feedforward"], conv_layout=True, use_conv_block=False, cross_attention=False, conv_kernel_size=3)
+            mm = M.Mimi(M.MimiConfig(channels=1, sample_rate=float(2 * hop * 12.5), frame_rate=12.5, renormalize=True, seanet=seanet, transformer=tr,
+                                     quantizer_nq=c["nq"], quantizer_bins=c["bins"], quantizer_dim=c["qdim"]))
+        P = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in tape.value(lambda: fill(mm))}
         mc = rng.integers(0, c["bins"], size=(2, c["nq"], int(rng.integers(1, 8))))
-        pcm = np.asarray(mm.decode(mx.array(mc)))
+        if tape.reference:
+            pcm = np.asarray(mm.decode(mx.array(mc)))
         opcm = OC.mimi_decode(P, torch.as_tensor(mc).long(), c).numpy()
-        assert pcm.shape == opcm.shape, (pcm.shape, opcm.shape)
-        errs.append(np.abs(pcm - opcm).max())
+        errs.append(tape.err(lambda: pcm, opcm))
         p_in = 0.5 * rng.standard_normal((2, 1, int(rng.integers(1, 5)) * 2 * hop + int(rng.integers(0, hop))))
-        assert np.array_equal(np.asarray(mm.encode(mx.array(p_in))), OC.mimi_encode(P, torch.as_tensor(p_in), c).numpy()), ("mimi encode", c)
+        assert np.array_equal(np.asarray(tape.value(lambda: np.asarray(mm.encode(mx.array(p_in))))), OC.mimi_encode(P, torch.as_tensor(p_in), c).numpy()), ("mimi encode", c)
         print("mimi ratios", ratios, "heads", heads, "context", c["context"], "nq", c["nq"], "ksize", c["ksize"], c["last_ksize"], "err", float(errs[-1]))
         worst = max(worst, float(max(errs)))
+    tape.close()
     assert worst < 1e-9, worst
     print("LIVE OK", worst)
 

@@ -76,11 +76,14 @@ def main():
 
 def live(n):
     """--live N: random STFT / iSTFT / mel-filterbank / log-mel configurations, the reference's dsp.py (float32, NumPy standing in for MLX)
-    vs oracle/dsp.py side by side."""
+    vs oracle/dsp.py side by side (--record / --replay: live_tape.py)."""
     sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
     from oracle import dsp as O
+    from live_tape import Tape
+    tape = Tape("dsp", n, sys.argv)
     numpy_mlx_shim.install()
-    dsp = load(os.path.join(REF, "dsp.py"), "ref_dsp_live")
+    if tape.reference:
+        dsp = load(os.path.join(REF, "dsp.py"), "ref_dsp_live")
     worst = {"stft": 0.0, "istft": 0.0, "mel": 0.0, "window": 0.0}
     for seed in range(n):
         rng = np.random.default_rng(5000 + seed)
@@ -92,35 +95,32 @@ def live(n):
         pad_mode = str(rng.choice(["reflect", "constant"]))
         x = rng.standard_normal(int(rng.integers(2 * n_fft, 6 * n_fft))).astype(np.float32)
         kw = dict(n_fft=n_fft, hop_length=hop, win_length=win_length, window=window, center=center, pad_mode=pad_mode)
-        a, b = np.asarray(dsp.stft(numpy_mlx_shim.array(x), **kw)), O.stft(x, **kw)
-        assert a.shape == b.shape, (kw, a.shape, b.shape)
-        worst["stft"] = max(worst["stft"], float(np.abs(a - b).max() / max(1.0, np.abs(b).max())))
+        b = O.stft(x, **kw)
+        worst["stft"] = max(worst["stft"], tape.err(lambda: dsp.stft(numpy_mlx_shim.array(x), **kw), b) / max(1.0, np.abs(b).max()))
         for size in (int(rng.integers(3, 40)),):
             for name in ("hanning", "hamming", "blackman", "bartlett"):
                 for periodic in (False, True):
-                    wa, wb = np.asarray(getattr(dsp, name)(size, periodic=periodic)), getattr(O, name)(size, periodic=periodic)
-                    worst["window"] = max(worst["window"], float(np.abs(wa - wb).max()))
+                    wb = getattr(O, name)(size, periodic=periodic)
+                    worst["window"] = max(worst["window"], tape.err(lambda: getattr(dsp, name)(size, periodic=periodic), wb))
         # iSTFT of a centred reflect STFT with a full-length window (the combination the reference's own callers use)
         nf = int(rng.choice([16, 64, 256]))
         hp = nf // int(rng.choice([2, 4]))
         y = rng.standard_normal(6 * nf).astype(np.float32)
-        spec = np.asarray(dsp.stft(numpy_mlx_shim.array(y), n_fft=nf, hop_length=hp))
+        spec = np.asarray(O.stft(y, n_fft=nf, hop_length=hp)).astype(np.complex64)       # both sides invert the same spectrogram
         norm = bool(rng.integers(0, 2))
-        ia = np.asarray(dsp.istft(numpy_mlx_shim.array(spec.T), hop_length=hp, win_length=nf, normalized=norm))
         ib = O.istft(spec.T, hop_length=hp, win_length=nf, normalized=norm)
-        ok = np.isfinite(ia)
-        assert ia.shape == ib.shape
-        worst["istft"] = max(worst["istft"], float(np.abs(ia[ok] - ib[ok]).max()))
+        worst["istft"] = max(worst["istft"], tape.err(lambda: dsp.istft(numpy_mlx_shim.array(spec.T), hop_length=hp, win_length=nf, normalized=norm), ib))
         sr = int(rng.choice([16000, 22050, 24000, 44100]))
         mk = dict(sample_rate=sr, n_fft=int(rng.choice([256, 400, 1024])), n_mels=int(rng.choice([20, 40, 80, 128])), f_min=float(rng.choice([0.0, 50.0])),
                   f_max=float(rng.choice([sr / 2, sr / 2 - 1000.0])), norm=[None, "slaney"][int(rng.integers(0, 2))], mel_scale=str(rng.choice(["htk", "slaney"])))
-        worst["mel"] = max(worst["mel"], float(np.abs(np.asarray(dsp.mel_filters(**mk)) - O.mel_filters(**mk)).max()))
+        worst["mel"] = max(worst["mel"], tape.err(lambda: dsp.mel_filters(**mk), O.mel_filters(**mk)))
         print("dsp", kw, "| istft", nf, hp, norm, "| mel", mk["sample_rate"], mk["n_mels"], mk["norm"], mk["mel_scale"])
     # interpolate (tts/models/interpolate.py): nearest / linear, align_corners on / off / None, up- and down-scaling incl. the 300x of Kokoro's source
     sys.path.insert(0, HERE)
     import numpy_mlx_nn as nn_shim
     core64, _ = nn_shim.install(precise=True)
-    interp = load(os.path.join(REF, "tts", "models", "interpolate.py"), "ref_interpolate_live")
+    if tape.reference:
+        interp = load(os.path.join(REF, "tts", "models", "interpolate.py"), "ref_interpolate_live")
     worst["interp"] = 0.0
     for seed in range(6 * n):
         rng = np.random.default_rng(6000 + seed)
@@ -133,10 +133,9 @@ def live(n):
             kw = dict(size=int(rng.integers(1, 900)))
         if x.shape[-1] * kw.get("scale_factor", 1.0) > 40000:
             x = x[..., :100]
-        a = np.asarray(interp.interpolate(core64.array(x), mode=mode, align_corners=ac, **kw))
         b = O.interpolate(x, mode=mode, align_corners=ac, **kw)
-        assert a.shape == np.asarray(b).shape, (x.shape, kw, mode, ac, a.shape, np.asarray(b).shape)
-        worst["interp"] = max(worst["interp"], float(np.abs(a - np.asarray(b)).max()))
+        worst["interp"] = max(worst["interp"], tape.err(lambda: interp.interpolate(core64.array(x), mode=mode, align_corners=ac, **kw), b))
+    tape.close()
     print(worst)
     assert worst["interp"] < 1e-12, worst
     assert worst["stft"] < 2e-4 and worst["istft"] < 5e-5 and worst["mel"] < 5e-6 and worst["window"] < 1e-6, worst

@@ -18,19 +18,20 @@ import numpy_mlx_nn as shim          # noqa: E402
 
 REF = "/root/reference/mlx_audio"
 mx, nn = shim.install(precise=True)
-for name, path in (("mlx_audio", REF), ("mlx_audio.tts", f"{REF}/tts"), ("mlx_audio.tts.models", f"{REF}/tts/models"),
-                   ("mlx_audio.tts.models.kokoro", f"{REF}/tts/models/kokoro")):
-    shim.stub_package(name, path)
-hub = types.ModuleType("huggingface_hub")
-hub.snapshot_download = hub.hf_hub_download = None
-sys.modules["huggingface_hub"] = hub
-import mlx_audio.dsp as _dsp          # noqa: E402
-u = types.ModuleType("mlx_audio.utils")
-u.load_audio = None
-for n in ("hanning", "mel_filters", "stft", "istft"):
-    setattr(u, n, getattr(_dsp, n))
-sys.modules["mlx_audio.utils"] = u
-from mlx_audio.tts.models.kokoro import kokoro as K          # noqa: E402
+if "--replay" not in sys.argv:                                 # replaying a --live record needs no reference source
+    for name, path in (("mlx_audio", REF), ("mlx_audio.tts", f"{REF}/tts"), ("mlx_audio.tts.models", f"{REF}/tts/models"),
+                       ("mlx_audio.tts.models.kokoro", f"{REF}/tts/models/kokoro")):
+        shim.stub_package(name, path)
+    hub = types.ModuleType("huggingface_hub")
+    hub.snapshot_download = hub.hf_hub_download = None
+    sys.modules["huggingface_hub"] = hub
+    import mlx_audio.dsp as _dsp          # noqa: E402
+    u = types.ModuleType("mlx_audio.utils")
+    u.load_audio = None
+    for n in ("hanning", "mel_filters", "stft", "istft"):
+        setattr(u, n, getattr(_dsp, n))
+    sys.modules["mlx_audio.utils"] = u
+    from mlx_audio.tts.models.kokoro import kokoro as K          # noqa: E402
 
 # The harmonic source's STFT phase (istftnet.py:473-505: arctan2(imag, real)) is ill-defined wherever a bin is exactly real -- DC,
 # Nyquist, and every bin of the reflect-symmetric first frame: there the imaginary part is FFT rounding noise (or a signed zero)
@@ -97,18 +98,22 @@ def live(n):
     oracle's forward; durations identical, waveform 1e-9."""
     import torch
     from oracle import kokoro as OK
+    from live_tape import Tape
+    tape = Tape("kokoro", n, sys.argv)
     OK.EFFECTIVE_WEIGHTS_BF16 = False
     cfg = json.loads(json.dumps(KOKORO_CONFIG))
     vocab = {chr(0x100 + i): i for i in range(cfg["n_token"])}
-    model = K.Model(K.ModelConfig(**cfg, vocab=vocab))
-    model.eval()
+    if tape.reference:
+        model = K.Model(K.ModelConfig(**cfg, vocab=vocab))
+        model.eval()
     worst = 0.0
     for seed in range(n):
         rng = np.random.default_rng(4000 + seed)
         P = synth.kokoro_weights(cfg, seed=int(rng.integers(1, 100)))
         P["predictor.F0_proj.weight"] = P["predictor.F0_proj.weight"] * float(rng.uniform(200, 900))
-        for k, v in P.items():
-            shim.set_parameter(model, k, v.double().numpy())
+        if tape.reference:
+            for k, v in P.items():
+                shim.set_parameter(model, k, v.double().numpy())
         n_ph, speed = int(rng.integers(3, 14)), float(rng.uniform(0.4, 1.2))
         ids = rng.integers(1, cfg["n_token"], size=n_ph)
         ref_s = rng.standard_normal((1, 256))
@@ -118,16 +123,22 @@ def live(n):
         def noise(shape):
             draws["noise"] = rng.standard_normal(shape)
             return draws["noise"]
-        mx.random.strict = True
-        mx.random.queue[:] = [("uniform", rand_ini), ("normal", noise), ("normal", lambda shape: np.zeros(shape))]
-        res = model("".join(chr(0x100 + int(i)) for i in ids), mx.array(ref_s), speed=speed, return_output=True)
-        mx.random.strict = False
+        if tape.reference:
+            mx.random.strict = True
+            mx.random.queue[:] = [("uniform", rand_ini), ("normal", noise), ("normal", lambda shape: np.zeros(shape))]
+            res = model("".join(chr(0x100 + int(i)) for i in ids), mx.array(ref_s), speed=speed, return_output=True)
+            mx.random.strict = False
+        shape = tape.value(lambda: draws["noise"].shape)
+        if not tape.reference:
+            noise(shape)                                       # the draw the reference's call made, from the same generator state
         audio, pd = OK.forward({k: v.double() for k, v in P.items()}, torch.as_tensor(np.concatenate([[0], ids, [0]]))[None], torch.as_tensor(ref_s), cfg,
                                speed=speed, rand_ini=torch.as_tensor(rand_ini), noise=torch.as_tensor(draws["noise"]))
-        assert np.array_equal(pd.numpy(), np.asarray(res.pred_dur)), (pd, res.pred_dur)
-        err = float(np.abs(audio.numpy().reshape(-1) - np.asarray(res.audio).reshape(-1)).max())
+        pred_dur = tape.value(lambda: np.asarray(res.pred_dur))
+        assert np.array_equal(pd.numpy(), np.asarray(pred_dur)), (pd, pred_dur)
+        err = tape.err(lambda: np.asarray(res.audio).reshape(-1), audio.numpy().reshape(-1), sample=512)
         worst = max(worst, err)
-        print("kokoro phonemes", n_ph, "speed", round(speed, 2), "durations", np.asarray(res.pred_dur).tolist(), "samples", np.asarray(res.audio).size, "err", err)
+        print("kokoro phonemes", n_ph, "speed", round(speed, 2), "durations", pred_dur, "samples", audio.numel(), "err", err)
+    tape.close()
     assert worst < 2e-8, worst          # float64 on both sides; the harmonic phase integrates over every frame, so the error grows with the
                                         # utterance (measured: 1.4e-9 at 58 frames, 3-6 frames per phoneme)
     print("LIVE OK", worst)

@@ -19,24 +19,25 @@ import synth_params                  # noqa: E402
 
 REF = "/root/reference/mlx_audio"
 mx, nn = shim.install(precise=True)
-for name, path in (("mlx_audio", REF), ("mlx_audio.lm", f"{REF}/lm"), ("mlx_audio.lm.models", f"{REF}/lm/models"), ("mlx_audio.tts", f"{REF}/tts"),
-                   ("mlx_audio.tts.models", f"{REF}/tts/models"), ("mlx_audio.tts.models.qwen3_tts", f"{REF}/tts/models/qwen3_tts"),
-                   ("mlx_audio.codec", f"{REF}/codec"), ("mlx_audio.codec.models", f"{REF}/codec/models"),
-                   ("mlx_audio.codec.models.mimi", f"{REF}/codec/models/mimi")):
-    shim.stub_package(name, path)
-for stub, names in (("huggingface_hub", ("snapshot_download", "hf_hub_download")),):
-    m = types.ModuleType(stub)
-    for n in names:
-        setattr(m, n, None)
-    sys.modules[stub] = m
-u = types.ModuleType("mlx_audio.utils")
-u.load_audio = None
-import mlx_audio.dsp as _dsp          # noqa: E402
-u.hanning, u.mel_filters, u.stft = _dsp.hanning, _dsp.mel_filters, _dsp.stft
-sys.modules["mlx_audio.utils"] = u
+if "--replay" not in sys.argv:                                 # replaying a --live record needs no reference source
+    for name, path in (("mlx_audio", REF), ("mlx_audio.lm", f"{REF}/lm"), ("mlx_audio.lm.models", f"{REF}/lm/models"), ("mlx_audio.tts", f"{REF}/tts"),
+                       ("mlx_audio.tts.models", f"{REF}/tts/models"), ("mlx_audio.tts.models.qwen3_tts", f"{REF}/tts/models/qwen3_tts"),
+                       ("mlx_audio.codec", f"{REF}/codec"), ("mlx_audio.codec.models", f"{REF}/codec/models"),
+                       ("mlx_audio.codec.models.mimi", f"{REF}/codec/models/mimi")):
+        shim.stub_package(name, path)
+    for stub, names in (("huggingface_hub", ("snapshot_download", "hf_hub_download")),):
+        m = types.ModuleType(stub)
+        for n in names:
+            setattr(m, n, None)
+        sys.modules[stub] = m
+    u = types.ModuleType("mlx_audio.utils")
+    u.load_audio = None
+    import mlx_audio.dsp as _dsp          # noqa: E402
+    u.hanning, u.mel_filters, u.stft = _dsp.hanning, _dsp.mel_filters, _dsp.stft
+    sys.modules["mlx_audio.utils"] = u
 
-from mlx_audio.tts.models.qwen3_tts import config as C            # noqa: E402
-from mlx_audio.tts.models.qwen3_tts import talker as T            # noqa: E402
+    from mlx_audio.tts.models.qwen3_tts import config as C            # noqa: E402
+    from mlx_audio.tts.models.qwen3_tts import talker as T            # noqa: E402
 
 CP = dict(vocab_size=80, hidden_size=48, intermediate_size=96, num_hidden_layers=2, num_attention_heads=4, num_key_value_heads=2, head_dim=16,
           num_code_groups=4)
@@ -374,7 +375,10 @@ def live(n):
     import torch
     sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
     from oracle import qwen3 as OQ
-    from mlx_audio.tts.models.qwen3_tts import speech_tokenizer as S
+    from live_tape import Tape
+    tape = Tape("qwen3", n, sys.argv)
+    if tape.reference:
+        from mlx_audio.tts.models.qwen3_tts import speech_tokenizer as S
     worst = 0.0
     for seed in range(n):
         rng = np.random.default_rng(2000 + seed)
@@ -398,27 +402,35 @@ def live(n):
               "mrope_section": sec, "num_code_groups": g, "codec_eos_token_id": 2150, "text_hidden_size": 24, "cp_vocab_size": cp["vocab_size"],
               "cp_hidden_size": cph, "cp_intermediate_size": 2 * cph, "cp_num_hidden_layers": cp["num_hidden_layers"], "cp_num_attention_heads": heads,
               "cp_num_key_value_heads": kv, "cp_head_dim": hd, "cp_rope_theta": 1000000.0}
-        talker = T.Qwen3TTSTalkerForConditionalGeneration(C.Qwen3TTSTalkerConfig(**tk))
-        P = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in fill(talker)}
+        if tape.reference:
+            talker = T.Qwen3TTSTalkerForConditionalGeneration(C.Qwen3TTSTalkerConfig(**tk))
+        P = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in tape.value(lambda: fill(talker))}
         bsz, s0 = int(rng.integers(1, 4)), int(rng.integers(2, 9))
         x = rng.standard_normal((bsz, s0, hidden))
-        cache, ocache = talker.make_cache(), OQ.make_cache(oc["num_hidden_layers"])
-        lg, _ = talker(mx.array(x), cache=cache)
+        ocache = OQ.make_cache(oc["num_hidden_layers"])
+        if tape.reference:
+            cache = talker.make_cache()
+            lg, _ = talker(mx.array(x), cache=cache)
         olg, _ = OQ.talker_forward(P, torch.as_tensor(x), ocache, cfg=oc)
-        errs = [np.abs(np.asarray(lg) - olg.numpy()).max()]
+        errs = [tape.err(lambda: lg, olg.numpy())]
         for _ in range(2):
             x1 = rng.standard_normal((bsz, 1, hidden))
-            lg, _ = talker(mx.array(x1), cache=cache)
+            if tape.reference:
+                lg, _ = talker(mx.array(x1), cache=cache)
             olg, _ = OQ.talker_forward(P, torch.as_tensor(x1), ocache, cfg=oc)
-            errs.append(np.abs(np.asarray(lg) - olg.numpy()).max())
-        cc, occ = talker.code_predictor.make_cache(), OQ.make_cache(oc["cp_num_hidden_layers"])
+            errs.append(tape.err(lambda: lg, olg.numpy()))
+        occ = OQ.make_cache(oc["cp_num_hidden_layers"])
+        if tape.reference:
+            cc = talker.code_predictor.make_cache()
         cx = rng.standard_normal((bsz, 2, hidden))
-        cl, cc, _ = talker.code_predictor(mx.array(cx), cache=cc, generation_step=0)
-        errs.append(np.abs(np.asarray(cl) - OQ.code_predictor_forward(P, torch.as_tensor(cx), occ, 0, oc).numpy()).max())
+        if tape.reference:
+            cl, cc, _ = talker.code_predictor(mx.array(cx), cache=cc, generation_step=0)
+        errs.append(tape.err(lambda: cl, OQ.code_predictor_forward(P, torch.as_tensor(cx), occ, 0, oc).numpy()))
         for st in range(1, g - 1):
             c1 = rng.standard_normal((bsz, 1, hidden))
-            cl, cc, _ = talker.code_predictor(mx.array(c1), cache=cc, generation_step=st)
-            errs.append(np.abs(np.asarray(cl) - OQ.code_predictor_forward(P, torch.as_tensor(c1), occ, st, oc).numpy()).max())
+            if tape.reference:
+                cl, cc, _ = talker.code_predictor(mx.array(c1), cache=cc, generation_step=st)
+            errs.append(tape.err(lambda: cl, OQ.code_predictor_forward(P, torch.as_tensor(c1), occ, st, oc).numpy()))
         # tokenizer decoder with other strides
         ups = [int(v) for v in rng.choice([2, 3, 4, 5], size=int(rng.integers(2, 4)))]
         rat = [int(v) for v in rng.choice([2, 3], size=int(rng.integers(1, 3)))]
@@ -432,19 +444,22 @@ def live(n):
                "layer_scale_initial_scale": 0.01, "head_dim": 8, "num_attention_heads": dh, "num_hidden_layers": td["num_hidden_layers"],
                "num_key_value_heads": dh, "num_quantizers": nq, "num_semantic_quantizers": 1, "rms_norm_eps": 1e-5, "rope_theta": 10000.0,
                "upsample_rates": ups, "upsampling_ratios": rat}
-        tok = S.Qwen3TTSSpeechTokenizer(C.Qwen3TTSTokenizerConfig(decoder_config=C.Qwen3TTSTokenizerDecoderConfig(**td)))
-        PT = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in fill(tok, rule=lambda nm: "small" if nm.endswith((".alpha", ".beta")) else None)}
+        if tape.reference:
+            tok = S.Qwen3TTSSpeechTokenizer(C.Qwen3TTSTokenizerConfig(decoder_config=C.Qwen3TTSTokenizerDecoderConfig(**td)))
+        names = tape.value(lambda: fill(tok, rule=lambda nm: "small" if nm.endswith((".alpha", ".beta")) else None))
+        PT = {k: torch.as_tensor(synth_params.value(k, sh, r)) for k, sh, r in names}
         codes = rng.integers(0, 32, size=(2, nq, int(rng.integers(2, 7))))
-        wav = np.asarray(tok.decoder(mx.array(codes)))
+        if tape.reference:
+            wav = np.asarray(tok.decoder(mx.array(codes)))
         owav = OQ.tokenizer_decode(PT, torch.as_tensor(codes), otd).numpy()
-        assert wav.shape == owav.shape, (wav.shape, owav.shape)
-        errs.append(np.abs(wav - owav).max())
+        errs.append(tape.err(lambda: wav, owav))
         worst = max(worst, float(max(errs)))
         print("qwen3 heads", heads, "kv", kv, "hd", hd, "mrope", sec, "groups", g, "| tokenizer ups", ups, rat, "nq", nq, "max err", float(max(errs)))
     # sampler chain (qwen3_tts.py:805-860 over lm/sample_utils.py): random logits and settings, the same injected uniform on both sides
-    from mlx_audio.tts.models.qwen3_tts import qwen3_tts as QM
-    m = QM.Model.__new__(QM.Model)
-    mx.random.strict = True
+    if tape.reference:
+        from mlx_audio.tts.models.qwen3_tts import qwen3_tts as QM
+        m = QM.Model.__new__(QM.Model)
+        mx.random.strict = True
     n_cases = 60 * n
     for case in range(n_cases):
         rng = np.random.default_rng(9000 + case)
@@ -458,12 +473,17 @@ def live(n):
         if sup is not None and len(sup) >= V:
             sup = sup[: V - 1]
         u = float(rng.random())
-        mx.random.queue[:] = [("categorical", np.array([u]))]
-        tok = int(np.asarray(m._sample_token(mx.array(logits[None, None, :]), generated_tokens=gen, suppress_tokens=sup, **kw))[0, 0])
-        mx.random.queue[:] = []
+
+        def ref_token():
+            mx.random.queue[:] = [("categorical", np.array([u]))]
+            t = int(np.asarray(m._sample_token(mx.array(logits[None, None, :]), generated_tokens=gen, suppress_tokens=sup, **kw))[0, 0])
+            mx.random.queue[:] = []
+            return t
+        tok = tape.value(ref_token)
         want = OQ.sample_token(torch.as_tensor(logits), u, kw["temperature"], kw["top_k"], kw["top_p"], kw["repetition_penalty"], gen, sup, kw["min_p"])
         assert tok == want, (case, kw, tok, want)
     mx.random.strict = False
+    tape.close()
     print("sampler cases identical:", n_cases)
     assert worst < 1e-9, worst
     print("LIVE OK", worst)

@@ -14,20 +14,21 @@ import synth_params                  # noqa: E402
 
 REF = "/root/reference/mlx_audio"
 mx, nn = shim.install(precise=True)
-for name, path in (("mlx_audio", REF), ("mlx_audio.stt", f"{REF}/stt"), ("mlx_audio.stt.models", f"{REF}/stt/models"),
-                   ("mlx_audio.stt.models.whisper", f"{REF}/stt/models/whisper")):
-    shim.stub_package(name, path)
-import types                          # noqa: E402
-for stub, names in (("mlx_audio.stt.utils", ("load_audio",)), ("huggingface_hub", ("snapshot_download",))):
-    m = types.ModuleType(stub)
-    for n in names:
-        setattr(m, n, None)
-    sys.modules[stub] = m
-import mlx_audio.dsp as _dsp          # noqa: E402  (the reference's dsp.py, through the shim)
-u = types.ModuleType("mlx_audio.utils")
-u.hanning, u.mel_filters, u.stft = _dsp.hanning, _dsp.mel_filters, _dsp.stft
-sys.modules["mlx_audio.utils"] = u
-from mlx_audio.stt.models.whisper import whisper as W     # noqa: E402
+if "--replay" not in sys.argv:                                 # replaying a --live record needs no reference source
+    for name, path in (("mlx_audio", REF), ("mlx_audio.stt", f"{REF}/stt"), ("mlx_audio.stt.models", f"{REF}/stt/models"),
+                       ("mlx_audio.stt.models.whisper", f"{REF}/stt/models/whisper")):
+        shim.stub_package(name, path)
+    import types                          # noqa: E402
+    for stub, names in (("mlx_audio.stt.utils", ("load_audio",)), ("huggingface_hub", ("snapshot_download",))):
+        m = types.ModuleType(stub)
+        for n in names:
+            setattr(m, n, None)
+        sys.modules[stub] = m
+    import mlx_audio.dsp as _dsp          # noqa: E402  (the reference's dsp.py, through the shim)
+    u = types.ModuleType("mlx_audio.utils")
+    u.hanning, u.mel_filters, u.stft = _dsp.hanning, _dsp.mel_filters, _dsp.stft
+    sys.modules["mlx_audio.utils"] = u
+    from mlx_audio.stt.models.whisper import whisper as W     # noqa: E402
 
 DIMS = dict(n_mels=80, n_audio_ctx=60, n_audio_state=64, n_audio_head=4, n_audio_layer=2, n_vocab=300, n_text_ctx=32, n_text_state=64,
             n_text_head=4, n_text_layer=2)
@@ -210,6 +211,8 @@ def live(n):
     import torch
     sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
     from oracle import whisper as OW
+    from live_tape import Tape
+    tape = Tape("whisper", n, sys.argv)
     worst = 0.0
     for seed in range(n):
         rng = np.random.default_rng(1000 + seed)
@@ -218,29 +221,35 @@ def live(n):
         d = dict(n_mels=int(rng.choice([16, 80])), n_audio_ctx=int(rng.integers(5, 40)), n_audio_state=state, n_audio_head=heads,
                  n_audio_layer=int(rng.integers(1, 4)), n_vocab=int(rng.integers(50, 200)), n_text_ctx=int(rng.integers(8, 24)), n_text_state=state,
                  n_text_head=heads, n_text_layer=int(rng.integers(1, 4)))
-        model = W.Model(W.ModelDimensions(**d), dtype=mx.float32)
-        names = [(k, v.shape) for k, v in shim.flat_parameters(model)]
-        for k, sh in names:
-            shim.set_parameter(model, k, synth_params.value(k, sh))
+        if tape.reference:
+            model = W.Model(W.ModelDimensions(**d), dtype=mx.float32)
+        names = tape.value(lambda: [(k, v.shape) for k, v in shim.flat_parameters(model)])
+        if tape.reference:
+            for k, sh in names:
+                shim.set_parameter(model, k, synth_params.value(k, sh))
         P = {k: torch.as_tensor(synth_params.value(k, sh)) for k, sh in names}
         b = int(rng.integers(1, 4))
         mel = rng.standard_normal((b, 2 * d["n_audio_ctx"], d["n_mels"]))
-        xa = model.encoder(mx.array(mel))
+        if tape.reference:
+            xa = model.encoder(mx.array(mel))
         oxa = OW.encoder(P, torch.as_tensor(mel), d)
         nt = int(rng.integers(1, d["n_text_ctx"] - 3))
         toks = rng.integers(0, d["n_vocab"], size=(b, nt))
-        lg, kv, _ = model.decoder(mx.array(toks), xa)
+        if tape.reference:
+            lg, kv, _ = model.decoder(mx.array(toks), xa)
         olg, cache = OW.decoder_forward(P, torch.as_tensor(toks), oxa, None, d)
-        errs = [np.abs(np.asarray(xa) - oxa.numpy()).max(), np.abs(np.asarray(lg) - olg.numpy()).max()]
+        errs = [tape.err(lambda: xa, oxa.numpy()), tape.err(lambda: lg, olg.numpy())]
         for _ in range(2):
             t1 = rng.integers(0, d["n_vocab"], size=(b, 1))
-            lg, kv, _ = model.decoder(mx.array(t1), xa, kv_cache=kv)
+            if tape.reference:
+                lg, kv, _ = model.decoder(mx.array(t1), xa, kv_cache=kv)
             olg, cache = OW.decoder_forward(P, torch.as_tensor(t1), oxa, cache, d)
-            errs.append(np.abs(np.asarray(lg) - olg.numpy()).max())
+            errs.append(tape.err(lambda: lg, olg.numpy()))
         worst = max(worst, float(max(errs)))
         print("whisper", d, "max err", float(max(errs)))
     # logit filters + greedy update on random logits under random token histories (decoding.py:307-442)
-    from mlx_audio.stt.models.whisper import decoding as D
+    if tape.reference:
+        from mlx_audio.stt.models.whisper import decoding as D
     tk = StubTokenizer()
     spec = OW.TokenizerSpec(eot=200, sot=201, no_timestamps=208, timestamp_begin=209, no_speech=207, blank_ids=(7,), language=202, task=203,
                             transcribe=203, translate=204, sot_lm=205, sot_prev=206)
@@ -257,17 +266,20 @@ def live(n):
             logits[:, T:] += float(rng.uniform(1, 6))
         sup = sorted(set(int(v) for v in rng.integers(0, 300, size=int(rng.integers(0, 6)))))
         mi = [None, 0, 2, 30][int(rng.integers(0, 4))]
-        filters = [D.SuppressBlank(tk, 3, 300)] + ([D.SuppressTokens(sup, 300)] if sup else []) + [D.ApplyTimestampRules(tk, 3, mi)]
-        y = mx.array(logits)
-        for f in filters:
-            y = f.apply(y, mx.array(toks))
+        if tape.reference:
+            filters = [D.SuppressBlank(tk, 3, 300)] + ([D.SuppressTokens(sup, 300)] if sup else []) + [D.ApplyTimestampRules(tk, 3, mi)]
+            y = mx.array(logits)
+            for f in filters:
+                y = f.apply(y, mx.array(toks))
+            y = np.asarray(y)
         want = OW.apply_filters(torch.as_tensor(logits), toks.tolist(), spec, 3, sup, max_initial_timestamp_index=mi).numpy()
-        y = np.asarray(y)
-        fin = np.isfinite(y)
-        assert np.array_equal(fin, np.isfinite(want)) and (not fin.any() or np.abs(y[fin] - want[fin]).max() < 1e-12), (case, toks.tolist(), sup, mi)
-        nt, comp, slp = D.GreedyDecoder(0.0, E).update(mx.array(toks), mx.array(y), mx.zeros(B))
+        assert tape.err(lambda: y, want, same_nonfinite=True) < 1e-12, (case, toks.tolist(), sup, mi)
+        if tape.reference:
+            nt, comp, slp = D.GreedyDecoder(0.0, E).update(mx.array(toks), mx.array(y), mx.zeros(B))
         ont, ocomp, oslp = OW.greedy_update(toks.tolist(), torch.as_tensor(want), torch.zeros(B, dtype=torch.float64), E)
-        assert np.array_equal(np.asarray(nt), np.array(ont)) and bool(comp) == ocomp and np.allclose(np.asarray(slp), oslp.numpy(), rtol=0, atol=1e-12, equal_nan=True), case
+        nt, comp, slp = tape.value(lambda: (np.asarray(nt), bool(comp), np.asarray(slp, dtype=np.float64)))
+        assert np.array_equal(np.asarray(nt), np.array(ont)) and comp == ocomp and np.allclose(np.asarray(slp), oslp.numpy(), rtol=0, atol=1e-12, equal_nan=True), case
+    tape.close()
     print("filter / greedy cases identical:", cases)
     assert worst < 1e-10, worst
     print("LIVE OK", worst)

@@ -1,6 +1,7 @@
-"""The committed fixtures under tests/golden/ are outputs of the reference's own source.  Where that source is present (the build
-container: /root/reference), every generator is re-run into a scratch directory and its output compared with the committed file --
-so a fixture can never drift from the code that is supposed to have produced it.  Skipped elsewhere (the GPU box has no /root/reference)."""
+"""The committed fixtures under tests/golden/ are outputs of the reference's own source.  Where that source is present (REF in the
+generators), every generator is re-run into a scratch directory and its output compared with the committed file -- so a fixture can
+never drift from the code that is supposed to have produced it; without it those tests skip.  The random-configuration comparisons
+of the oracle with the reference run everywhere, against the reference results recorded in tests/golden/*_live_golden.npz."""
 import json
 import os
 import subprocess
@@ -54,14 +55,15 @@ def test_fixture_is_what_the_reference_code_produces(generator, tmp_path):
             assert np.array_equal(a, b), k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/mlx_audio"), reason="the reference source is only present in the build container")
 @pytest.mark.parametrize("generator,n", [("make_dsp_golden.py", 12), ("make_whisper_golden.py", 4), ("make_qwen3_golden.py", 4), ("make_codec_golden.py", 5), ("make_kokoro_golden.py", 2)])
 def test_oracle_agrees_with_the_reference_code_on_random_configurations(generator, n):
     """Beyond the committed fixtures: ``--live N`` draws N random configurations (head counts, GQA ratios, MRoPE sections, code-book counts,
     stride lists, depthwise / noise switches, attention contexts, kernel sizes; for Kokoro random utterances, styles, speeds and weight
     seeds), runs the reference's classes through the NumPy stand-in and the oracle side by side, and requires 1e-9 (identical integer
     results).  This is what guards the oracle's generality between the small fixture configurations and the full-size ones the CUDA path is
-    tested against; it found two hard-coded assumptions (decoder layer indices for four upsampling stages, SNAC's depthwise stem)."""
-    r = subprocess.run([sys.executable, os.path.join(HERE, generator), "--live", str(n)], cwd=ROOT, env=dict(os.environ, OMP_NUM_THREADS="4"),
+    tested against; it found two hard-coded assumptions (decoder layer indices for four upsampling stages, SNAC's depthwise stem).
+    ``--replay`` draws the same configurations and runs the oracle against the reference's results as ``--live N --record`` stored them
+    (tests/golden/live_tape.py), so it needs no reference source."""
+    r = subprocess.run([sys.executable, os.path.join(HERE, generator), "--live", str(n), "--replay"], cwd=ROOT, env=dict(os.environ, OMP_NUM_THREADS="4"),
                        capture_output=True, text=True, timeout=900)
     assert r.returncode == 0 and "LIVE OK" in r.stdout, (r.stdout[-1500:], r.stderr[-1500:])
